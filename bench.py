@@ -13,6 +13,8 @@ A "step" is one packet wave: every resident stream encodes one 40 ms / 16 kHz pa
   cpu_baseline : the unmodified reference (oracle/_ref: FIX encoder + FLP decoder) on all host cores, bounded sample
 
 `--impl reference` times only that CPU baseline and prints the same JSON shape.
+`--dump-outputs DIR` also writes what the last timed step of both paths returned, for a fixed sample of the streams
+(see dump_outputs), so that two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -287,6 +289,23 @@ def bind_to_gpu_numa(index):
     return "not bound"
 
 
+DUMP_STREAMS = 8192   # 2 paths x 8192 streams x (128 + 2 + 640 + 1) float32 values = 51 MB
+
+
+def dump_outputs(out_dir, torch, n_streams, paths):
+    """Write the last timed step's outputs of each path as <path>_<name>.npy (float32), rows of a fixed seeded sample of
+    the streams (stream_index.npy, float64).  Payload bytes past the payload's length are not part of the result and
+    are written as 0."""
+    os.makedirs(out_dir, exist_ok=True)
+    rows = np.sort(np.random.default_rng(0).choice(n_streams, min(n_streams, DUMP_STREAMS), replace=False))
+    np.save(os.path.join(out_dir, "stream_index.npy"), rows.astype(np.float64))
+    for path, arrays in paths.items():
+        got = {k: t.index_select(0, torch.as_tensor(rows, device=t.device)).cpu().numpy() for k, t in arrays.items()}
+        got["payload"][np.arange(CAP)[None, :] >= got["nbytes"][:, :1]] = 0
+        for k, a in got.items():
+            np.save(os.path.join(out_dir, "%s_%s.npy" % (path, k)), a.astype(np.float32))
+
+
 def emit(line):
     """The one JSON line goes to the process's original stdout; everything else that libraries print to file descriptor 1
     (NCCL's version banner, for instance) was redirected to stderr at start-up."""
@@ -309,6 +328,7 @@ def main():
     ap.add_argument("--streams", type=int, default=65536, help="streams per GPU")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-root-ingest", action="store_true", help="skip the single-ingest-point measurement (N > 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs (rank 0's streams) to DIR")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "solo_b200" else args.warmup
 
@@ -435,6 +455,11 @@ def main():
     checksum = int(h_out.to(torch.int64).sum().item())
     h2d = world * N * (1280 + CAP + 4 + 4)      # whole job, per step: PCM in (encoder) + payload, lengths, flags in (decoder)
     d2h = world * N * (CAP + 4 + 1280 + 4)      # payload + lengths out (encoder) + PCM, return codes out (decoder)
+
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, torch, N, {
+            "device": {"payload": d_bits, "nbytes": d_nb, "pcm": d_out, "ret": d_ret},
+            "e2e": {"payload": h_bits, "nbytes": h_nb, "pcm": h_out, "ret": h_ret}})
 
     if rank == 0:
         peak, peak_src = measured_peaks()

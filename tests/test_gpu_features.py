@@ -3,7 +3,8 @@
 import numpy as np
 import pytest
 
-from tests.util import load_clip, load_golden, loss_flags, speech_replay, trim_payload
+from tests.util import (RowDigests, assert_matches_reference, enc_row, load_clip, load_golden, loss_flags, speech_replay,
+                        trim_payload)
 
 pytestmark = pytest.mark.gpu
 
@@ -130,52 +131,63 @@ def test_loss_trimming_on_device_matches_the_receiver_restatement(sb):
     eb.close(); db.close(); db_ref.close()
 
 
+CONFIG2 = dict(N=4096, T=50, cap=160)
+
+
+def config2_sample(N):
+    return sorted(set(list(range(0, N, 67)) + [1, 2, 3, N - 1]))[:64]
+
+
 def test_config2_batch_4096_streams_50_packets_sampled_against_reference(sb):
     """BASELINE config 2: 4 096 concurrent streams, encode only, 50 packets (2 s).  Every stream runs on the GPU; 64 of
-    them (spread over the batch, all four input gains) are replayed through libjc1_fix.so and must match byte for byte."""
-    from oracle import ref
-    if not ref.available():
-        pytest.skip("oracle/_ref not built")
-    N, T, cap = 4096, 50, 160
+    them (spread over the batch, all four input gains) must match libjc1_fix.so byte for byte."""
+    N, T, cap = CONFIG2["N"], CONFIG2["T"], CONFIG2["cap"]
     clip = load_clip()
-    sample = sorted(set(list(range(0, N, 67)) + [1, 2, 3, N - 1]))[:64]
-    refs = {s: ref.RefEncoder("fix", rate=13600) for s in sample}
+    sample = config2_sample(N)
     eb = sb.EncoderBatch(N, rate=13600)
+    enc = RowDigests(T, len(sample))
     for p in range(T):
         x = speech_replay(clip, N, 1, first_packet=p)[0]
         bits, nb = eb.encode(x, cap=cap)
         assert (nb[:, 0] <= cap).all()
-        for s in sample:
-            b, rnb, n = refs[s].encode(x[s])
-            assert tuple(nb[s]) == rnb and bytes(bits[s, :n]) == b, (p, s)
+        for i, s in enumerate(sample):
+            enc.add(p, i, enc_row(bits[s, :nb[s, 0]], nb[s]))
     eb.close()
+    assert_matches_reference("features_config2", enc=enc)
 
 
-def test_config5_full_batch_with_per_stream_loss_sampled_against_reference(sb):
-    """BASELINE configs 3 + 5 at full size: 65 536 streams, encode -> receiver-side trimming on the device -> decode with
-    a 50 % loss process per stream (seed 1 + stream id, dec_main.c:229-241); 48 sampled streams against libjc1_flp.so fed
-    the same payloads and flags (PCM identical; the north star allows +-1 LSB)."""
-    import torch
-    from oracle import ref
-    if not ref.available():
-        pytest.skip("oracle/_ref not built")
-    N, T, cap = 65536, 8, 128
-    clip = load_clip()
+CONFIG5 = dict(N=65536, T=8, cap=128)
+
+
+def config5_sample_and_flags(N, T):
+    """48 sampled streams with a 50 % loss process each (seed 1 + stream id, dec_main.c:229-241); arbitrary flags for
+    everybody else."""
     sample = [0, 1, 2, 3] + list(range(997, N, 1489))[:44]
     flags = np.full((N, T), 4, np.int32)
     for s in sample:
         flags[s] = loss_flags(T, 50, seed=1 + s)
     rng = np.random.Generator(np.random.PCG64(7))
-    other = rng.integers(1, 5, size=(N, T)).astype(np.int32)       # everybody else: arbitrary flags
+    other = rng.integers(1, 5, size=(N, T)).astype(np.int32)
     mask = np.ones(N, bool); mask[sample] = False
     flags[mask] = other[mask]
+    return sample, flags
+
+
+def test_config5_full_batch_with_per_stream_loss_sampled_against_reference(sb):
+    """BASELINE configs 3 + 5 at full size: 65 536 streams, encode -> receiver-side trimming on the device -> decode with
+    a 50 % loss process per stream; 48 sampled streams against libjc1_flp.so fed the same payloads and flags (PCM
+    identical; the north star allows +-1 LSB)."""
+    import torch
+    N, T, cap = CONFIG5["N"], CONFIG5["T"], CONFIG5["cap"]
+    clip = load_clip()
+    sample, flags = config5_sample_and_flags(N, T)
     dev = torch.device("cuda", 0)
     eb, db = sb.EncoderBatch(N), sb.DecoderBatch(N)
-    rdec = {s: ref.RefDecoder("flp") for s in sample}
     d_bits, d_nb = torch.zeros((N, cap), dtype=torch.uint8, device=dev), torch.zeros((N, 2), dtype=torch.int16, device=dev)
     d_tb, d_tnb = torch.zeros_like(d_bits), torch.zeros_like(d_nb)
     d_pcm, d_ret = torch.zeros((N, 640), dtype=torch.int16, device=dev), torch.zeros(N, dtype=torch.int32, device=dev)
     st = torch.cuda.current_stream().cuda_stream
+    pcm_d = RowDigests(T, len(sample))
     for p in range(T):
         x = torch.from_numpy(speech_replay(clip, N, 1, first_packet=p)[0]).to(dev)
         f = torch.from_numpy(flags[:, p].copy()).to(dev)
@@ -185,13 +197,11 @@ def test_config5_full_batch_with_per_stream_loss_sampled_against_reference(sb):
         torch.cuda.synchronize()
         assert int((d_ret != 0).sum().item()) == 0
         idx = torch.tensor(sample, device=dev)
-        bits, nb, pcm = d_bits[idx].cpu().numpy(), d_nb[idx].cpu().numpy(), d_pcm[idx].cpu().numpy()
-        for i, s in enumerate(sample):
-            pb, pnb = trim_payload(bytes(bits[i, :nb[i, 0]]), nb[i], int(flags[s, p]))
-            want, r = rdec[s].decode(pb, pnb, int(flags[s, p]))
-            assert r == 0
-            assert np.abs(pcm[i].astype(np.int32) - want.astype(np.int32)).max() <= 0, (p, s, int(flags[s, p]))
+        pcm = d_pcm[idx].cpu().numpy()
+        for i in range(len(sample)):
+            pcm_d.add(p, i, pcm[i].tobytes())
     eb.close(); db.close()
+    assert_matches_reference("features_config5", pcm=pcm_d)
 
 
 def test_single_stream_small_output_buffer(sb):
@@ -207,42 +217,46 @@ def test_single_stream_small_output_buffer(sb):
         e.close()
 
 
+PACKETS_20MS = dict(N=130, T=40, cap=128, sample=[0, 1, 64, 65, 129])
+
+
+def packets_20ms_inputs(clip, N, T):
+    """[T, N, 320] windows of the clip at per-stream offsets, and a 40 % loss process per stream (seed 3 + stream id)."""
+    off = (np.arange(N) * 7919 * 320) % (len(clip) - 320 * (T + 1))
+    x = np.stack([np.stack([clip[o + p * 320:o + (p + 1) * 320] for o in off]) for p in range(T)]).astype(np.int16)
+    flags = np.array([loss_flags(T, 40, seed=3 + s) for s in range(N)], np.int32)
+    return x, flags
+
+
 def test_20ms_packets_on_device(sb):
     """framesize_ms = 20 through the batched ABI and the drop-in ABI against the reference (FIX bytes, FLP PCM)."""
-    from oracle import ref
-    if not ref.available():
-        pytest.skip("oracle/_ref not built")
-    N, T, cap = 130, 40, 128
+    N, T, cap, sample = PACKETS_20MS["N"], PACKETS_20MS["T"], PACKETS_20MS["cap"], PACKETS_20MS["sample"]
     clip = load_clip()
     eb, db = sb.EncoderBatch(N, rate=13600, framesize_ms=20), sb.DecoderBatch(N, framesize_ms=20)
-    sample = [0, 1, 64, 65, 129]
-    renc = {s: ref.RefEncoder("fix", rate=13600, framesize_ms=20) for s in sample}
-    rdec = {s: ref.RefDecoder("flp", framesize_ms=20) for s in sample}
-    off = (np.arange(N) * 7919 * 320) % (len(clip) - 320 * (T + 1))
-    flags = np.array([loss_flags(T, 40, seed=3 + s) for s in range(N)], np.int32)
+    x, flags = packets_20ms_inputs(clip, N, T)
+    enc, pcm_d = RowDigests(T, len(sample)), RowDigests(T, len(sample))
     for p in range(T):
-        x = np.stack([clip[o + p * 320:o + (p + 1) * 320] for o in off]).astype(np.int16)
-        bits, nb = eb.encode(x, cap=cap)
+        bits, nb = eb.encode(x[p], cap=cap)
         tb, tnb = np.zeros_like(bits), np.zeros_like(nb)
         for s in range(N):
             pb, pnb = trim_payload(bytes(bits[s, :nb[s, 0]]), nb[s], flags[s, p])
             tb[s, :len(pb)] = np.frombuffer(pb, np.uint8); tnb[s] = pnb
         pcm, ret = db.decode(tb, tnb, flags[:, p].copy())
         assert pcm.shape == (N, 320) and (ret == 0).all()
-        for s in sample:
-            b, rnb, n = renc[s].encode(x[s])
-            assert tuple(nb[s]) == rnb and bytes(bits[s, :n]) == b, (p, s)
-            want, r = rdec[s].decode(bytes(tb[s, :tnb[s, 0]]), tuple(tnb[s]), int(flags[s, p]))
-            assert np.array_equal(pcm[s], want), (p, s)
+        for i, s in enumerate(sample):
+            enc.add(p, i, enc_row(bits[s, :nb[s, 0]], nb[s]))
+            pcm_d.add(p, i, pcm[s].tobytes())
     eb.close(); db.close()
     e, d = sb.SoloEncoder(rate=13600, framesize_ms=20), sb.SoloDecoder(framesize_ms=20)
-    r0 = ref.RefEncoder("fix", rate=13600, framesize_ms=20)
+    single = RowDigests(10, 1)
     for p in range(10):
         b, nb2, n = e.encode(clip[p * 320:(p + 1) * 320])
-        assert (b, nb2, n) == r0.encode(clip[p * 320:(p + 1) * 320])
+        assert n == len(b)
+        single.add(p, 0, enc_row(b, nb2))
         y, r = d.decode(b, nb2, 4)
         assert r == 0 and y.size == 320 and d.last_nsamples == 320
     e.close(); d.close()
+    assert_matches_reference("features_20ms", enc=enc, pcm=pcm_d, single=single)
 
 
 def test_example_file_codec_reproduces_the_reference_cli_files(sb, tmp_path):
@@ -266,18 +280,20 @@ def test_example_file_codec_reproduces_the_reference_cli_files(sb, tmp_path):
         assert hashlib.md5(out.read_bytes()).hexdigest() == str(g[key]), key
 
 
+JOINT = dict(N=67, T=20, cap=192, sample=[0, 1, 33, 66])
+
+
+def joint_flags(N, T):
+    return np.array([loss_flags(T, 40, seed=11 + s) for s in range(N)], np.int32)
+
+
 def test_joint_mode1_on_device(sb):
     """The reference's joint mode 1 through the batched ABI and the drop-in ABI (unsupported modes are refused)."""
-    from oracle import ref
-    if not ref.available():
-        pytest.skip("oracle/_ref not built")
-    N, T, cap = 67, 20, 192
+    N, T, cap, sample = JOINT["N"], JOINT["T"], JOINT["cap"], JOINT["sample"]
     x = speech_replay(load_clip(), N, T)
     eb, db = sb.EncoderBatch(N, rate=13600, joint_hb=1), sb.DecoderBatch(N, joint_hb=1)
-    sample = [0, 1, 33, 66]
-    renc = {s: ref.RefEncoder("fix", rate=13600, joint_hb=1) for s in sample}
-    rdec = {s: ref.RefDecoder("flp", joint_hb=1) for s in sample}
-    flags = np.array([loss_flags(T, 40, seed=11 + s) for s in range(N)], np.int32)
+    flags = joint_flags(N, T)
+    enc, pcm_d = RowDigests(T, len(sample)), RowDigests(T, len(sample))
     for p in range(T):
         bits, nb = eb.encode(x[p], cap=cap)
         tb, tnb = np.zeros_like(bits), np.zeros_like(nb)
@@ -286,16 +302,17 @@ def test_joint_mode1_on_device(sb):
             tb[s, :len(pb)] = np.frombuffer(pb, np.uint8); tnb[s] = pnb
         pcm, ret = db.decode(tb, tnb, flags[:, p].copy())
         assert (ret == 0).all()
-        for s in sample:
-            b, rnb, n = renc[s].encode(x[p, s])
-            assert tuple(nb[s]) == rnb and bytes(bits[s, :n]) == b, (p, s)
-            want, r = rdec[s].decode(bytes(tb[s, :tnb[s, 0]]), tuple(tnb[s]), int(flags[s, p]))
-            assert np.array_equal(pcm[s], want), (p, s)
+        for i, s in enumerate(sample):
+            enc.add(p, i, enc_row(bits[s, :nb[s, 0]], nb[s]))
+            pcm_d.add(p, i, pcm[s].tobytes())
     eb.close(); db.close()
     e = sb.SoloEncoder(rate=13600, joint_enable=1, joint_mode=1)
     b, nb2, n = e.encode(x[0, 0])
-    assert (b, nb2, n) == ref.RefEncoder("fix", rate=13600, joint_hb=1).encode(x[0, 0])
+    assert n == len(b)
+    single = RowDigests(1, 1)
+    single.add(0, 0, enc_row(b, nb2))
     e.close()
+    assert_matches_reference("features_joint_mode1", enc=enc, pcm=pcm_d, single=single)
     for bad in (dict(joint_enable=1, joint_mode=0), dict(joint_enable=1, joint_mode=2), dict(samplerate=32000), dict(framesize_ms=60)):
         with pytest.raises(sb.SoloError):
             sb.SoloEncoder(**bad)

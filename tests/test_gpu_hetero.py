@@ -1,18 +1,16 @@
 """Batched parity with *different* signal classes in neighbouring streams (SURVEY.md 8(d) ii/iii): the warps of a block, the
 two lane groups of a quantiser warp and the 64 threads of an entropy-coding / decoder block then take different paths
 (voiced / unvoiced, different decision delays, rewhitening, DTX-like silence, clipping) at the same time.
-Every row is compared with the unmodified reference run per stream: payload bytes + length fields against libjc1_fix.so,
-decoded PCM under a per-stream 50 % loss process against libjc1_flp.so fed the same payloads and flags.
+Every row is compared with the unmodified reference run per stream (digests in tests/golden/reference_digests.npz): payload
+bytes + length fields against libjc1_fix.so, decoded PCM under a per-stream 50 % loss process against libjc1_flp.so fed
+the same payloads and flags.
 Tolerances: payloads bit-exact; PCM 0 LSB (the north star allows +-1)."""
-from concurrent.futures import ThreadPoolExecutor
-
 import numpy as np
 import pytest
 
-from tests.util import load_clip, loss_flags, speech_replay, trim_payload
+from tests.util import RowDigests, assert_matches_reference, enc_row, load_clip, loss_flags, speech_replay, trim_payload
 
 pytestmark = pytest.mark.gpu
-PCM_TOL = 0
 
 
 @pytest.fixture(scope="module")
@@ -20,14 +18,6 @@ def sb():
     import solo_b200
     solo_b200.lib()
     return solo_b200
-
-
-@pytest.fixture(scope="module")
-def ref():
-    from oracle import ref as r
-    if not r.available():
-        pytest.skip("oracle/_ref not built")
-    return r
 
 
 def signal_classes(clip, n_rows, n_packets, seed=5):
@@ -60,70 +50,61 @@ def signal_classes(clip, n_rows, n_packets, seed=5):
     return np.ascontiguousarray(out.reshape(n_rows, n_packets, 640).transpose(1, 0, 2))
 
 
-def run_against_reference(sb, ref, x, rate, loss_perc=50, workers=16):
-    """x: [T, N, 640].  GPU batch vs one reference encoder + decoder per row (driven by a thread pool: the reference is
-    plain C behind ctypes, which releases the GIL)."""
+def hetero_flags(N, T, loss_perc=50):
+    flags = np.array([loss_flags(T, loss_perc, seed=1 + s) for s in range(N)], np.int32)
+    flags[::5] = 4           # every fifth row loss-free
+    return flags
+
+
+def run_against_reference(sb, case, x, rate):
+    """x: [T, N, 640].  GPU batch vs the reference run per row (one encoder + decoder per row, digests of its outputs
+    under `case`)."""
     T, N, _ = x.shape
     cap = 1024 if rate > 40000 else 256
     eb, db = sb.EncoderBatch(N, rate=rate), sb.DecoderBatch(N)
-    renc = [ref.RefEncoder("fix", rate=rate) for _ in range(N)]
-    rdec = [ref.RefDecoder("flp") for _ in range(N)]
-    flags = np.array([loss_flags(T, loss_perc, seed=1 + s) for s in range(N)], np.int32)
-    flags[::5] = 4           # every fifth row loss-free
-
-    def ref_row(args):
-        s, p = args
-        b, rnb, n = renc[s].encode(x[p, s])
-        f = int(flags[s, p])
-        if rnb[0] <= 0:      # DTX packet: nothing is sent, the receiver conceals
-            pb, pnb, f = bytes(16), (16, 8), 1
-        else:
-            pb, pnb = trim_payload(b, rnb, f)
-        y, r = rdec[s].decode(pb, pnb, f)
-        return b, rnb, n, pb, pnb, f, y, r
-
-    with ThreadPoolExecutor(workers) as pool:
-        for p in range(T):
-            bits, nb = eb.encode(x[p], cap=cap)
-            rows = list(pool.map(ref_row, [(s, p) for s in range(N)]))
-            dbits = np.zeros((N, cap), np.uint8)
-            dnb = np.zeros((N, 2), np.int16)
-            f_eff = np.zeros(N, np.int32)
-            want = np.zeros((N, 640), np.int16)
-            for s, (b, rnb, n, pb, pnb, f, y, r) in enumerate(rows):
-                assert tuple(nb[s]) == rnb, ("length fields", p, s, s % 8)
-                assert bytes(bits[s, :max(n, 0)]) == b[:max(n, 0)], ("payload", p, s, s % 8)
-                assert r == 0
-                dbits[s, :len(pb)] = np.frombuffer(pb, np.uint8)
-                dnb[s] = pnb
-                f_eff[s] = f
-                want[s] = y
-            pcm, ret = db.decode(dbits, dnb, f_eff)
-            assert (ret == 0).all()
-            d = np.abs(pcm.astype(np.int32) - want.astype(np.int32)).max(axis=1)
-            assert d.max() <= PCM_TOL, ("pcm", p, int(d.argmax()), int(d.argmax()) % 8, int(d.max()))
-    for o in renc + rdec:
-        o.close()
+    flags = hetero_flags(N, T)
+    enc, pcm_d = RowDigests(T, N), RowDigests(T, N)
+    for p in range(T):
+        bits, nb = eb.encode(x[p], cap=cap)
+        dbits = np.zeros((N, cap), np.uint8)
+        dnb = np.zeros((N, 2), np.int16)
+        f_eff = np.zeros(N, np.int32)
+        for s in range(N):
+            b = bytes(bits[s, :max(int(nb[s, 0]), 0)])
+            enc.add(p, s, enc_row(b, nb[s]))
+            f = int(flags[s, p])
+            if nb[s, 0] <= 0:    # DTX packet: nothing is sent, the receiver conceals
+                pb, pnb, f = bytes(16), (16, 8), 1
+            else:
+                pb, pnb = trim_payload(b, nb[s], f)
+            dbits[s, :len(pb)] = np.frombuffer(pb, np.uint8)
+            dnb[s] = pnb
+            f_eff[s] = f
+        pcm, ret = db.decode(dbits, dnb, f_eff)
+        assert (ret == 0).all()
+        for s in range(N):
+            pcm_d.add(p, s, pcm[s].tobytes())
     eb.close(); db.close()
+    assert_matches_reference(case, enc=enc, pcm=pcm_d)
 
 
-def test_neighbouring_streams_of_eight_signal_classes_match_the_reference(sb, ref):
+def test_neighbouring_streams_of_eight_signal_classes_match_the_reference(sb):
     x = signal_classes(load_clip(), 256, 40)
-    run_against_reference(sb, ref, x, rate=13600)
+    run_against_reference(sb, "hetero_classes", x, rate=13600)
 
 
 @pytest.mark.parametrize("rate", [6000, 24000, 100000])
-def test_signal_classes_at_other_rates(sb, ref, rate):
+def test_signal_classes_at_other_rates(sb, rate):
     x = signal_classes(load_clip(), 64, 20, seed=rate)
-    run_against_reference(sb, ref, x, rate=rate)
+    run_against_reference(sb, "hetero_rate%d" % rate, x, rate=rate)
 
 
-def test_full_batch_sample_of_1024_streams_25_packets(sb, ref):
-    """BASELINE configs 3 + 5 at full size (65 536 streams, per-stream loss process, trimming on the device): 1 024 streams
-    spread over the batch x 25 packets against the reference (SURVEY.md 8(d) config 4 wording)."""
-    import torch
-    N, T, cap = 65536, 25, 128
-    clip = load_clip()
+FULL_BATCH = dict(N=65536, T=25, cap=128)
+
+
+def full_batch_sample_and_flags(N, T):
+    """1 024 sampled streams spread over the batch (per-stream loss process, seed 1 + stream id) and arbitrary flags for
+    every other stream."""
     sample = sorted(set(list(range(0, N, 64))))[:1024]
     flags = np.full((N, T), 4, np.int32)
     for s in sample:
@@ -132,40 +113,36 @@ def test_full_batch_sample_of_1024_streams_25_packets(sb, ref):
     other = rng.integers(1, 5, size=(N, T)).astype(np.int32)
     mask = np.ones(N, bool); mask[sample] = False
     flags[mask] = other[mask]
+    return sample, flags
+
+
+def test_full_batch_sample_of_1024_streams_25_packets(sb):
+    """BASELINE configs 3 + 5 at full size (65 536 streams, per-stream loss process, trimming on the device): 1 024 streams
+    spread over the batch x 25 packets against the reference (SURVEY.md 8(d) config 4 wording)."""
+    import torch
+    N, T, cap = FULL_BATCH["N"], FULL_BATCH["T"], FULL_BATCH["cap"]
+    clip = load_clip()
+    sample, flags = full_batch_sample_and_flags(N, T)
     dev = torch.device("cuda", 0)
     eb, db = sb.EncoderBatch(N), sb.DecoderBatch(N)
-    renc = {s: ref.RefEncoder("fix", rate=13600) for s in sample}
-    rdec = {s: ref.RefDecoder("flp") for s in sample}
     d_bits, d_nb = torch.zeros((N, cap), dtype=torch.uint8, device=dev), torch.zeros((N, 2), dtype=torch.int16, device=dev)
     d_tb, d_tnb = torch.zeros_like(d_bits), torch.zeros_like(d_nb)
     d_pcm, d_ret = torch.zeros((N, 640), dtype=torch.int16, device=dev), torch.zeros(N, dtype=torch.int32, device=dev)
     st = torch.cuda.current_stream().cuda_stream
     idx = torch.tensor(sample, device=dev)
-
-    def ref_row(args):
-        s, p, xs = args
-        b, rnb, n = renc[s].encode(xs)
-        f = int(flags[s, p])
-        pb, pnb = trim_payload(b, rnb, f)
-        y, r = rdec[s].decode(pb, pnb, f)
-        return b, rnb, n, y, r
-
-    with ThreadPoolExecutor(32) as pool:
-        for p in range(T):
-            xh = speech_replay(clip, N, 1, first_packet=p)[0]
-            x = torch.from_numpy(xh).to(dev)
-            f = torch.from_numpy(flags[:, p].copy()).to(dev)
-            eb.encode_device(x.data_ptr(), d_bits.data_ptr(), cap, d_nb.data_ptr(), st)
-            sb.apply_loss_device(d_bits.data_ptr(), d_nb.data_ptr(), f.data_ptr(), d_tb.data_ptr(), d_tnb.data_ptr(), cap, N, st)
-            db.decode_device(d_pcm.data_ptr(), d_tb.data_ptr(), cap, d_tnb.data_ptr(), f.data_ptr(), d_ret.data_ptr(), st)
-            rows = list(pool.map(ref_row, [(s, p, xh[s]) for s in sample]))
-            torch.cuda.synchronize()
-            assert int((d_ret != 0).sum().item()) == 0
-            bits, nb, pcm = d_bits[idx].cpu().numpy(), d_nb[idx].cpu().numpy(), d_pcm[idx].cpu().numpy()
-            for i, s in enumerate(sample):
-                b, rnb, n, y, r = rows[i]
-                assert r == 0 and tuple(nb[i]) == rnb and bytes(bits[i, :n]) == b, (p, s)
-                assert np.abs(pcm[i].astype(np.int32) - y.astype(np.int32)).max() <= PCM_TOL, (p, s, int(flags[s, p]))
-    for o in list(renc.values()) + list(rdec.values()):
-        o.close()
+    enc, pcm_d = RowDigests(T, len(sample)), RowDigests(T, len(sample))
+    for p in range(T):
+        xh = speech_replay(clip, N, 1, first_packet=p)[0]
+        x = torch.from_numpy(xh).to(dev)
+        f = torch.from_numpy(flags[:, p].copy()).to(dev)
+        eb.encode_device(x.data_ptr(), d_bits.data_ptr(), cap, d_nb.data_ptr(), st)
+        sb.apply_loss_device(d_bits.data_ptr(), d_nb.data_ptr(), f.data_ptr(), d_tb.data_ptr(), d_tnb.data_ptr(), cap, N, st)
+        db.decode_device(d_pcm.data_ptr(), d_tb.data_ptr(), cap, d_tnb.data_ptr(), f.data_ptr(), d_ret.data_ptr(), st)
+        torch.cuda.synchronize()
+        assert int((d_ret != 0).sum().item()) == 0
+        bits, nb, pcm = d_bits[idx].cpu().numpy(), d_nb[idx].cpu().numpy(), d_pcm[idx].cpu().numpy()
+        for i in range(len(sample)):
+            enc.add(p, i, enc_row(bits[i, :nb[i, 0]], nb[i]))
+            pcm_d.add(p, i, pcm[i].tobytes())
     eb.close(); db.close()
+    assert_matches_reference("hetero_full_batch", enc=enc, pcm=pcm_d)

@@ -1,5 +1,6 @@
 """On-device parity: the sm_100a kernels, called through the C ABI of libsolo_b200.so, against
- (a) the committed golden vectors and (b) the unmodified reference (oracle/_ref) run on the same inputs.
+ (a) the committed golden vectors and (b) the unmodified reference's outputs on the same inputs (digests in
+ tests/golden/reference_digests.npz).
 Bar: encoder payloads + length fields byte-identical to the reference FIX build; decoded PCM identical (tolerance
 stated by the north star is +-1 LSB; we require 0) to the reference FLP build."""
 import hashlib
@@ -8,7 +9,8 @@ import struct
 import numpy as np
 import pytest
 
-from tests.util import load_clip, load_golden, loss_flags, speech_replay, synth_inputs, trim_payload
+from tests.util import (RowDigests, assert_matches_reference, enc_row, load_clip, load_golden, loss_flags, speech_replay,
+                        synth_inputs, trim_payload)
 
 pytestmark = pytest.mark.gpu
 
@@ -20,14 +22,6 @@ def sb():
     import solo_b200
     solo_b200.lib()
     return solo_b200
-
-
-@pytest.fixture(scope="module")
-def ref():
-    from oracle import ref as r
-    if not r.available():
-        pytest.skip("oracle/_ref not built")
-    return r
 
 
 def bitfile(pk):
@@ -81,49 +75,58 @@ def test_synthetic_inputs_golden(sb):
         assert hashlib.md5(bitfile(pk)).hexdigest() == str(g["synth_" + name]), name
 
 
-def test_batch_encode_matches_reference(sb, ref):
+BATCH_ENCODE = dict(N=256, T=12, cap=256)
+
+
+def test_batch_encode_matches_reference(sb):
     """Config 2 (reduced for test time): N streams x T packets of the speech-replay batch, every payload byte and both
     length fields equal to libjc1_fix.so run per stream."""
-    N, T, cap = 256, 12, 256
+    N, T, cap = BATCH_ENCODE["N"], BATCH_ENCODE["T"], BATCH_ENCODE["cap"]
     x = speech_replay(load_clip(), N, T)
     eb = sb.EncoderBatch(N, rate=13600)
-    refs = [ref.RefEncoder("fix", rate=13600) for _ in range(N)]
+    enc = RowDigests(T, N)
     for p in range(T):
         bits, nb = eb.encode(x[p], cap=cap)
         for s in range(N):
-            b, rnb, n = refs[s].encode(x[p, s])
-            assert tuple(nb[s]) == rnb, (p, s)
-            assert bytes(bits[s, :n]) == b, (p, s)
+            enc.add(p, s, enc_row(bits[s, :nb[s, 0]], nb[s]))
     eb.close()
+    assert_matches_reference("parity_batch_encode", enc=enc)
 
 
-def test_batch_roundtrip_with_loss_matches_reference(sb, ref):
+def roundtrip_flags(N, T):
+    flags = np.array([loss_flags(T, 50, seed=1 + s) for s in range(N)], np.int32)  # [N, T]
+    flags[:N // 4] = 4  # a quarter of the streams loss-free
+    return flags
+
+
+BATCH_ROUNDTRIP = dict(N=96, T=14, cap=256)
+
+
+def test_batch_roundtrip_with_loss_matches_reference(sb):
     """Config 3 + 5 (reduced): encode -> decode with a per-stream loss process (seed 1 + stream id, 50 %), PCM against
     libjc1_flp.so driven with identical flags."""
-    N, T, cap = 96, 14, 256
+    N, T, cap = BATCH_ROUNDTRIP["N"], BATCH_ROUNDTRIP["T"], BATCH_ROUNDTRIP["cap"]
     x = speech_replay(load_clip(), N, T)
     eb = sb.EncoderBatch(N)
     db = sb.DecoderBatch(N)
-    rdec = [ref.RefDecoder("flp") for _ in range(N)]
-    flags = np.array([loss_flags(T, 50, seed=1 + s) for s in range(N)], np.int32)  # [N, T]
-    flags[:N // 4] = 4  # a quarter of the streams loss-free
+    flags = roundtrip_flags(N, T)
+    pcm_d = RowDigests(T, N)
     for p in range(T):
         bits, nb = eb.encode(x[p], cap=cap)
         dbits = np.zeros((N, cap), np.uint8)
         dnb = np.zeros((N, 2), np.int16)
-        want = np.zeros((N, 640), np.int16)
         for s in range(N):
             b = bytes(bits[s, :nb[s, 0]])
             pb, pnb = trim_payload(b, nb[s], flags[s, p])
             dbits[s, :len(pb)] = np.frombuffer(pb, np.uint8)
             dnb[s] = pnb
-            want[s], r = rdec[s].decode(pb, pnb, flags[s, p])
-            assert r == 0
         pcm, ret = db.decode(dbits, dnb, flags[:, p].copy())
         assert (ret == 0).all()
-        assert np.abs(pcm.astype(np.int32) - want.astype(np.int32)).max() <= PCM_TOL, p
+        for s in range(N):
+            pcm_d.add(p, s, pcm[s].tobytes())
     eb.close()
     db.close()
+    assert_matches_reference("parity_batch_roundtrip", pcm=pcm_d)
 
 
 def test_full_size_properties(sb):

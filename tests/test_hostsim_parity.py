@@ -1,5 +1,6 @@
-"""Kernel arithmetic on the CPU: solo_b200/csrc/*.cuh compiled by g++ (tests/hostsim) against the golden fixtures and,
-where oracle/_ref is built, against the unmodified reference on inputs the fixtures do not cover.
+"""Kernel arithmetic on the CPU: solo_b200/csrc/*.cuh compiled by g++ (tests/hostsim) against the golden fixtures and
+against the unmodified reference's outputs on inputs the fixtures do not cover (digests in
+tests/golden/reference_digests.npz).
 
 The headers are written once as __host__ __device__ code, so what passes here is the same source nvcc compiles into
 libsolo_b200.so (the warp-per-stream quantiser sb_nsq_warp.cuh is device-only; its scalar model sb_nsq.cuh runs here and
@@ -11,7 +12,8 @@ import struct
 import numpy as np
 import pytest
 
-from tests.util import load_clip, load_golden, loss_flags, speech_replay, synth_inputs, trim_payload
+from tests.util import (RowDigests, assert_matches_reference, enc_row, load_clip, load_golden, loss_flags, speech_replay,
+                        synth_inputs, trim_payload)
 
 PCM_TOL = 0
 
@@ -85,41 +87,39 @@ def test_empty_and_error_inputs(sim):
     d.close()
 
 
-@pytest.fixture(scope="module")
-def ref():
-    from oracle import ref as r
-    if not r.available():
-        pytest.skip("oracle/_ref not built")
-    return r
-
-
-def test_speech_replay_streams_match_reference(sim, ref):
-    """SURVEY.md 8(d) batch (i), 12 streams x 30 packets, each stream with its own loss pattern (seed 1 + s, 50 %):
-    encoder bytes vs FIX, decoder PCM vs FLP fed the same payloads and flags."""
+def run_speech_replay_streams(Enc, Dec):
+    """SURVEY.md 8(d) batch (i), 12 streams x 30 packets, each stream with its own loss pattern (seed 1 + s, 50 %).
+    Enc / Dec: encoder and decoder classes with the call shapes of tests/hostsim/sim.py (the reference's too)."""
     S, P = 12, 30
     x = speech_replay(load_clip(), S, P)
+    enc, pcm = RowDigests(P, S), RowDigests(P, S)
     for s in range(S):
-        e_ref, e_sim = ref.RefEncoder("fix", rate=13600), sim.SimEncoder(rate=13600)
-        d_ref, d_sim = ref.RefDecoder("flp"), sim.SimDecoder()
+        e, d = Enc(rate=13600), Dec()
         flags = loss_flags(P, 50, seed=1 + s)
         for p in range(P):
-            b0, nb0, n0 = e_ref.encode(x[p, s])
-            b1, nb1, n1 = e_sim.encode(x[p, s])
-            assert (b0[:n0], nb0, n0) == (b1[:n1], nb1, n1), (s, p)
-            pb, pnb = trim_payload(b0, nb0, flags[p])
-            y0, r0 = d_ref.decode(pb, pnb, flags[p])
-            y1, r1 = d_sim.decode(pb, pnb, flags[p])
-            assert r0 == r1 == 0
-            assert np.abs(y0.astype(np.int32) - y1.astype(np.int32)).max() <= PCM_TOL, (s, p, flags[p])
-        for o in (e_ref, e_sim, d_ref, d_sim):
-            o.close()
+            b, nb, n = e.encode(x[p, s])
+            enc.add(p, s, enc_row(b[:max(n, 0)], nb) + struct.pack("<i", n))
+            pb, pnb = trim_payload(b, nb, flags[p])
+            y, r = d.decode(pb, pnb, flags[p])
+            assert r == 0, (s, p)
+            pcm.add(p, s, y.tobytes())
+        e.close(); d.close()
+    return dict(enc=enc, pcm=pcm)
 
 
-def test_random_rates_and_signals_match_reference(sim, ref):
-    """Seeded sweep over target rates and signal classes that the fixtures do not hold."""
+def test_speech_replay_streams_match_reference(sim):
+    """Encoder bytes vs FIX, decoder PCM vs FLP fed the same payloads and flags."""
+    assert_matches_reference("hostsim_speech_replay", **run_speech_replay_streams(sim.SimEncoder, sim.SimDecoder))
+
+
+def run_random_rates_and_signals(Enc, Dec):
+    """Seeded sweep over target rates and signal classes that the fixtures do not hold: 5 configurations x 4 signals
+    (one digest column each) x 25 packets."""
     rng = np.random.Generator(np.random.PCG64(99))
     clip = load_clip()
     t = np.arange(640 * 25)
+    enc, pcm = RowDigests(25, 20), RowDigests(25, 20)
+    col = 0
     for rate, mdi, dtx in ((8000, 0, 0), (11000, 1, 0), (13600, 0, 1), (20000, 0, 0), (40000, 1, 1)):
         off = int(rng.integers(0, len(clip) - 640 * 25))
         sigs = [clip[off:off + 640 * 25],
@@ -127,107 +127,107 @@ def test_random_rates_and_signals_match_reference(sim, ref):
                 (6000 * np.sin(2 * np.pi * (80 + 3e-3 * t) * t / 16000)).astype(np.int16),
                 np.clip(rng.normal(0, 500, 640 * 25), -32768, 32767).astype(np.int16)]
         for x in sigs:
-            a = encode(lambda **kw: ref.RefEncoder("fix", **kw), x, rate=rate, dtx=dtx, use_md_index=mdi)
-            b = encode(sim.SimEncoder, x, rate=rate, dtx=dtx, use_md_index=mdi)
-            assert [(p[0][:max(p[2], 0)], p[1], p[2]) for p in a] == [(p[0][:max(p[2], 0)], p[1], p[2]) for p in b], (rate, mdi, dtx)
-            d0, d1 = ref.RefDecoder("flp", use_md_index=mdi), sim.SimDecoder(use_md_index=mdi)
-            for (pb, nb, n) in a:
+            e, d = Enc(rate=rate, dtx=dtx, use_md_index=mdi), Dec(use_md_index=mdi)
+            for p in range(25):
+                b, nb, n = e.encode(x[p * 640:(p + 1) * 640])
+                enc.add(p, col, enc_row(b[:max(n, 0)], nb) + struct.pack("<i", n))
                 if nb[0] <= 0:        # DTX: nothing was sent, the receiver conceals
-                    y0, _ = d0.decode(bytes(16), (16, 8), 1)
-                    y1, _ = d1.decode(bytes(16), (16, 8), 1)
+                    y, _ = d.decode(bytes(16), (16, 8), 1)
                 else:
-                    y0, _ = d0.decode(pb[:n], nb, 4)
-                    y1, _ = d1.decode(pb[:n], nb, 4)
-                assert np.abs(y0.astype(np.int32) - y1.astype(np.int32)).max() <= PCM_TOL
-            d0.close(); d1.close()
+                    y, _ = d.decode(b[:n], nb, 4)
+                pcm.add(p, col, y.tobytes())
+            e.close(); d.close()
+            col += 1
+    return dict(enc=enc, pcm=pcm)
 
 
-def test_small_output_buffer_matches_reference(sim, ref):
+def test_random_rates_and_signals_match_reference(sim):
+    assert_matches_reference("hostsim_random_rates", **run_random_rates_and_signals(sim.SimEncoder, sim.SimDecoder))
+
+
+SMALL_CAPS = (100, 64, 16, 9, 4)
+
+
+def test_small_output_buffer_matches_reference(sim):
     """AGR_Sate_Buf_Size smaller than the packet (AGR_BWE_bits.c:166-168): the return value is min(cap, total), the length
-    fields still describe the whole packet, bytes past the cap are left alone."""
-    import ctypes as C
+    fields still describe the whole packet, and the first min(cap, total) bytes are the reference's."""
     clip = load_clip()
-    for cap in (100, 64, 16, 9, 4):
-        e, s = ref.RefEncoder("fix", rate=24000), sim.SimEncoder(rate=24000, cap=cap)
+    enc = RowDigests(12, len(SMALL_CAPS))
+    for i, cap in enumerate(SMALL_CAPS):
+        s = sim.SimEncoder(rate=24000, cap=cap)
         for p in range(12):
-            pcm = np.ascontiguousarray(clip[p * 640:(p + 1) * 640])
-            bits = (C.c_uint8 * 1024)()
-            C.memset(bits, 0xAA, 1024)
-            nb = (C.c_int16 * 6)()
-            n = e.L.AGR_Sate_Encoder_Encode(e.h, pcm.ctypes.data, bits, cap, nb)
             s.out[:] = 0xAA
-            b2, nb2, n2 = s.encode(pcm)
-            assert n == n2 == min(cap, nb[0]) and (nb[0], nb[1]) == nb2
-            assert bytes(bits[:n]) == bytes(s.out[:n]) and bytes(bits[cap:cap + 8]) == b"\xaa" * 8
-        e.close(); s.close()
+            b, nb, n = s.encode(clip[p * 640:(p + 1) * 640])
+            assert n == min(cap, nb[0]), (cap, p)
+            enc.add(p, i, enc_row(b, nb) + struct.pack("<i", n))
+        s.close()
+    assert_matches_reference("hostsim_small_output_buffer", enc=enc)
 
 
-def test_20ms_packets_match_reference(sim, ref):
-    """The reference's other packet size (framesize_ms = 20: one SILK frame + one high-band frame per packet, 4 high-band
-    bytes, AGR_BWE_SDK_API.c:78-81,106-110): payloads vs FIX, PCM vs FLP, with loss, DTX and the MD index flag."""
+def run_20ms_packets(Enc, Dec):
     clip = load_clip()
-    for rate, dtx, mdi in ((13600, 0, 0), (8000, 0, 1), (24000, 1, 0)):
-        e0 = ref.RefEncoder("fix", rate=rate, dtx=dtx, use_md_index=mdi, framesize_ms=20)
-        e1 = sim.SimEncoder(rate=rate, dtx=dtx, use_md_index=mdi, framesize_ms=20)
-        d0, d1 = ref.RefDecoder("flp", use_md_index=mdi, framesize_ms=20), sim.SimDecoder(use_md_index=mdi, framesize_ms=20)
+    enc, pcm = RowDigests(240, 3), RowDigests(240, 3)
+    for i, (rate, dtx, mdi) in enumerate(((13600, 0, 0), (8000, 0, 1), (24000, 1, 0))):
+        e = Enc(rate=rate, dtx=dtx, use_md_index=mdi, framesize_ms=20)
+        d = Dec(use_md_index=mdi, framesize_ms=20)
         flags = loss_flags(240, 30, seed=5)
         for p in range(240):
-            x = clip[p * 320:(p + 1) * 320]
-            b0, nb0, n0 = e0.encode(x)
-            b1, nb1, n1 = e1.encode(x)
-            assert (b0[:max(n0, 0)], nb0, n0) == (b1[:max(n1, 0)], nb1, n1), (rate, p)
-            if nb0[0] > 0:
-                assert nb0[1] >= 4 and n0 == nb0[0]
-                pb, pnb, f = trim_payload(b0, nb0, flags[p]) + (flags[p],)
+            b, nb, n = e.encode(clip[p * 320:(p + 1) * 320])
+            enc.add(p, i, enc_row(b[:max(n, 0)], nb) + struct.pack("<i", n))
+            if nb[0] > 0:
+                assert nb[1] >= 4 and n == nb[0], (rate, p)
+                pb, pnb, f = trim_payload(b, nb, flags[p]) + (flags[p],)
             else:                                   # DTX: nothing was sent
                 pb, pnb, f = bytes(16), (16, 8), 1
-            y0, r0 = d0.decode(pb, pnb, f)
-            y1, r1 = d1.decode(pb, pnb, f)
-            assert r0 == r1 == 0 and y0.size == y1.size == 320
-            assert np.abs(y0.astype(np.int32) - y1.astype(np.int32)).max() <= PCM_TOL, (rate, p, f)
-        for o in (e0, e1, d0, d1):
-            o.close()
+            y, r = d.decode(pb, pnb, f)
+            assert r == 0 and y.size == 320, (rate, p, f)
+            pcm.add(p, i, y.tobytes())
+        e.close(); d.close()
+    return dict(enc=enc, pcm=pcm)
 
 
-def test_joint_mode1_matches_reference(sim, ref):
-    """joint_enable = 1, joint_mode = 1 (AGR_BWE_SDK_API.c:63-66): one 40 ms high-band frame (4 bytes, 80-sample
-    sub-frames) per packet, core rate = target - 800."""
+def test_20ms_packets_match_reference(sim):
+    """The reference's other packet size (framesize_ms = 20: one SILK frame + one high-band frame per packet, 4 high-band
+    bytes, AGR_BWE_SDK_API.c:78-81,106-110): payloads vs FIX, PCM vs FLP, with loss, DTX and the MD index flag."""
+    assert_matches_reference("hostsim_20ms", **run_20ms_packets(sim.SimEncoder, sim.SimDecoder))
+
+
+def run_joint_mode1(Enc, Dec):
     clip = load_clip()
-    for rate, dtx, mdi in ((13600, 0, 0), (8000, 0, 1), (24000, 1, 0)):
-        e0 = ref.RefEncoder("fix", rate=rate, dtx=dtx, use_md_index=mdi, joint_hb=1)
-        e1 = sim.SimEncoder(rate=rate, dtx=dtx, use_md_index=mdi, joint_hb=1)
-        d0, d1 = ref.RefDecoder("flp", use_md_index=mdi, joint_hb=1), sim.SimDecoder(use_md_index=mdi, joint_hb=1)
+    enc, pcm = RowDigests(120, 3), RowDigests(120, 3)
+    for i, (rate, dtx, mdi) in enumerate(((13600, 0, 0), (8000, 0, 1), (24000, 1, 0))):
+        e = Enc(rate=rate, dtx=dtx, use_md_index=mdi, joint_hb=1)
+        d = Dec(use_md_index=mdi, joint_hb=1)
         flags = loss_flags(120, 30, seed=9)
         for p in range(120):
-            x = clip[p * 640:(p + 1) * 640]
-            b0, nb0, n0 = e0.encode(x)
-            b1, nb1, n1 = e1.encode(x)
-            assert (b0[:max(n0, 0)], nb0, n0) == (b1[:max(n1, 0)], nb1, n1), (rate, p)
-            if nb0[0] > 0:
-                pb, pnb, f = trim_payload(b0, nb0, flags[p]) + (flags[p],)
+            b, nb, n = e.encode(clip[p * 640:(p + 1) * 640])
+            enc.add(p, i, enc_row(b[:max(n, 0)], nb) + struct.pack("<i", n))
+            if nb[0] > 0:
+                pb, pnb, f = trim_payload(b, nb, flags[p]) + (flags[p],)
             else:
                 pb, pnb, f = bytes(16), (16, 8), 1
-            y0, r0 = d0.decode(pb, pnb, f)
-            y1, r1 = d1.decode(pb, pnb, f)
-            assert r0 == r1 == 0
-            assert np.abs(y0.astype(np.int32) - y1.astype(np.int32)).max() <= PCM_TOL, (rate, p, f)
-        for o in (e0, e1, d0, d1):
-            o.close()
+            y, r = d.decode(pb, pnb, f)
+            assert r == 0, (rate, p, f)
+            pcm.add(p, i, y.tobytes())
+        e.close(); d.close()
+    return dict(enc=enc, pcm=pcm)
 
 
-def test_long_run_with_level_changes_dtx_and_loss_bursts(sim, ref):
-    """Soak: 1 000 packets per configuration (40 ms, 20 ms, joint mode 1) of programme material that changes level, goes
-    silent (DTX on) and suffers loss bursts -- counters, hysteresis, CNG and concealment state must track the reference
-    packet after packet."""
+def test_joint_mode1_matches_reference(sim):
+    """joint_enable = 1, joint_mode = 1 (AGR_BWE_SDK_API.c:63-66): one 40 ms high-band frame (4 bytes, 80-sample
+    sub-frames) per packet, core rate = target - 800."""
+    assert_matches_reference("hostsim_joint_mode1", **run_joint_mode1(sim.SimEncoder, sim.SimDecoder))
+
+
+def run_long_run(Enc, Dec):
     clip = load_clip()
     rng = np.random.Generator(np.random.PCG64(5))
-    for rate, dtx, mdi, fs, j in ((13600, 1, 0, 40, 0), (9000, 0, 1, 20, 0), (20000, 1, 0, 40, 1)):
+    P = 1000
+    enc, pcm = RowDigests(P, 3), RowDigests(P, 3)
+    for i, (rate, dtx, mdi, fs, j) in enumerate(((13600, 1, 0, 40, 0), (9000, 0, 1, 20, 0), (20000, 1, 0, 40, 1))):
         spp = 16 * fs
-        kw = dict(rate=rate, dtx=dtx, use_md_index=mdi, framesize_ms=fs, joint_hb=j)
-        e0, e1 = ref.RefEncoder("fix", **kw), sim.SimEncoder(**kw)
-        d0 = ref.RefDecoder("flp", use_md_index=mdi, framesize_ms=fs, joint_hb=j)
-        d1 = sim.SimDecoder(use_md_index=mdi, framesize_ms=fs, joint_hb=j)
-        P = 1000
+        e = Enc(rate=rate, dtx=dtx, use_md_index=mdi, framesize_ms=fs, joint_hb=j)
+        d = Dec(use_md_index=mdi, framesize_ms=fs, joint_hb=j)
         flags = loss_flags(P, 25, seed=77)
         pos, gain = 0, 1.0
         for p in range(P):
@@ -236,19 +236,25 @@ def test_long_run_with_level_changes_dtx_and_loss_bursts(sim, ref):
             seg = clip[pos:pos + spp]
             pos = (pos + spp) % (len(clip) - spp)
             x = np.clip(seg.astype(np.float64) * gain, -32768, 32767).astype(np.int16)
-            b0, nb0, n0 = e0.encode(x)
-            b1, nb1, n1 = e1.encode(x)
-            assert (b0[:max(n0, 0)], nb0, n0) == (b1[:max(n1, 0)], nb1, n1), (rate, p)
+            b, nb, n = e.encode(x)
+            enc.add(p, i, enc_row(b[:max(n, 0)], nb) + struct.pack("<i", n))
             f = flags[p] if (p // 200) % 2 == 0 else (1 if rng.random() < 0.6 else 4)
-            if nb0[0] <= 0:
+            if nb[0] <= 0:
                 pb, pnb, f = bytes(16), (16, 8), 1
             else:
-                pb, pnb = trim_payload(b0, nb0, f)
-            y0, r0 = d0.decode(pb, pnb, f)
-            y1, r1 = d1.decode(pb, pnb, f)
-            assert r0 == r1 == 0 and np.abs(y0.astype(np.int32) - y1.astype(np.int32)).max() <= PCM_TOL, (rate, p, f)
-        for o in (e0, e1, d0, d1):
-            o.close()
+                pb, pnb = trim_payload(b, nb, f)
+            y, r = d.decode(pb, pnb, f)
+            assert r == 0, (rate, p, f)
+            pcm.add(p, i, y.tobytes())
+        e.close(); d.close()
+    return dict(enc=enc, pcm=pcm)
+
+
+def test_long_run_with_level_changes_dtx_and_loss_bursts(sim):
+    """Soak: 1 000 packets per configuration (40 ms, 20 ms, joint mode 1) of programme material that changes level, goes
+    silent (DTX on) and suffers loss bursts -- counters, hysteresis, CNG and concealment state must track the reference
+    packet after packet."""
+    assert_matches_reference("hostsim_long_run", **run_long_run(sim.SimEncoder, sim.SimDecoder))
 
 
 def test_cooperative_analysis_under_32_lane_emulation(sim):

@@ -1,10 +1,14 @@
-"""Shared helpers of the test-suite (input synthesis, the reference driver's loss process, payload trimming)."""
+"""Shared helpers of the test-suite (input synthesis, the reference driver's loss process, payload trimming, digests of
+the reference's outputs)."""
+import hashlib
 import os
+import struct
 
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 GOLDEN = os.path.join(HERE, "golden")
+REFERENCE_DIGESTS = os.path.join(GOLDEN, "reference_digests.npz")
 
 
 def load_clip():
@@ -13,6 +17,44 @@ def load_clip():
 
 def load_golden():
     return np.load(os.path.join(GOLDEN, "golden.npz"))
+
+
+def enc_row(payload, nb):
+    """What an encoder call hands back for one stream: both length fields and the payload bytes."""
+    return struct.pack("<hh", int(nb[0]), int(nb[1])) + bytes(payload)
+
+
+class RowDigests:
+    """md5 of every (packet, stream) row of a run, folded into one digest per packet and one per stream.
+
+    tests/golden/make_reference_digests.py ran the unmodified reference on the inputs of the parity tests and stored the
+    folded digests in reference_digests.npz, so the tests compare byte for byte with the reference without needing it,
+    and a mismatch still names the packets and streams that differ."""
+
+    def __init__(self, n_packets, n_streams):
+        self.rows = np.zeros((n_packets, n_streams, 16), np.uint8)
+
+    def add(self, p, s, row):
+        self.rows[p, s] = np.frombuffer(hashlib.md5(row).digest(), np.uint8)
+
+    def folded(self):
+        fold = lambda rows: np.frombuffer(hashlib.md5(np.ascontiguousarray(rows).tobytes()).digest(), np.uint8)
+        return (np.stack([fold(self.rows[p]) for p in range(self.rows.shape[0])]),
+                np.stack([fold(self.rows[:, s]) for s in range(self.rows.shape[1])]))
+
+
+def assert_matches_reference(case, **digests):
+    """digests: kind ('enc', 'pcm', ...) -> RowDigests of this run; compared with the reference's digests of `case`."""
+    g = np.load(REFERENCE_DIGESTS)
+    for kind, d in sorted(digests.items()):
+        packets, streams = d.folded()
+        key = "%s:%s" % (case, kind)
+        want_p, want_s = g[key + ":packets"], g[key + ":streams"]
+        assert packets.shape == want_p.shape and streams.shape == want_s.shape, (key, packets.shape, want_p.shape)
+        bad_p = np.nonzero((packets != want_p).any(axis=1))[0]
+        bad_s = np.nonzero((streams != want_s).any(axis=1))[0]
+        assert len(bad_p) == 0 and len(bad_s) == 0, "%s differs from the reference in packets %s and streams %s" % (
+            key, bad_p[:20].tolist(), bad_s[:20].tolist())
 
 
 def _lcg(s):
